@@ -3,6 +3,8 @@
 
     python bench.py --gpus N --steps K --warmup W            (our CUDA path; N>1 under torchrun)
     python bench.py --impl reference --gpus N --steps K ...   (CPU reference arm: the oracle on host cores)
+    python bench.py ... --dump-outputs DIR                    (also writes the last timed step's chunk records as .npy,
+                                                               so that two builds can be compared on the same inputs)
 
 A "step" is one pass of the hot path (K1 scan -> K2 resolve -> K3 SHA-256 -> K4 probe) over one
 batch = BASELINE config[1]: 1024 x 64 MiB synthetic files per GPU, resident in HBM, generated on
@@ -110,6 +112,23 @@ def instr_ceiling(sm_total, sm_mhz, value_gbs):
             "source": "profiles/r02_sass_mix.txt (SASS count), profiles/r01_microbench.txt (64 thread-ops/clk/SM)"}
 
 
+DUMP_LIMIT = 64_000_000   # bytes of array data --dump-outputs writes at most
+
+
+def dump_outputs(out_dir, rec, known):
+    """Writes the chunk records of one step as DIR/<field>.npy: row (index in the step's record list), stream and end_off
+    as float64, digest (n x 32 bytes) and known as float32.  Above DUMP_LIMIT a fixed, seeded sample of rows is written."""
+    n = len(rec)
+    cap = DUMP_LIMIT // (3 * 8 + 32 * 4 + 4)
+    rows = np.arange(n) if n <= cap else np.sort(np.random.default_rng(0).choice(n, cap, replace=False))
+    r = rec[rows]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("row", rows.astype(np.float64)), ("stream", r["stream"].astype(np.float64)),
+                    ("end_off", r["end_off"].astype(np.float64)), ("digest", r["digest"].astype(np.float32)),
+                    ("known", (np.asarray(known)[rows] != 0).astype(np.float32))):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def union_ms(intervals):
     """Total length of the union of [t0,t1] intervals (ms)."""
     tot, cur0, cur1 = 0.0, None, None
@@ -176,8 +195,10 @@ def run_reference(args, rank: int, world: int):
         oracle.chunk_digest_streams(cfg, files[:threads], threads=threads)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        oracle.chunk_digest_streams(cfg, files, threads=threads)
+        rec = oracle.chunk_digest_streams(cfg, files, threads=threads)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rec, rec["flags"] & 1)
     val = n_sample * file_len * args.steps / dt / GIB
     sample = (f"{n_sample} x {args.file_mib} MiB files of the cfg2 corpus per step, one stream per task on "
               f"{threads} threads (best of {cpu_thread_candidates(cores)} on {cores} logical CPUs)")
@@ -516,6 +537,8 @@ def run_ours(args, rank: int, local_rank: int, world: int):
                            for t in timings]
     # ---- untimed post-run parity check (VERDICT r1 next-1a): the record list of the LAST timed step equals the oracle's
     last_rec = results[-1][0]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_rec, results[-1][2])
     if world == 1 and not args.no_verify and not reduced and args.avg_kib == 4096:
         import oracle
         t0 = time.perf_counter()
@@ -816,7 +839,13 @@ def main():
                          "stream slots then queue them FIFO per stream, which keeps the GPU fed without the host)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the chunk records of the last timed step (rank 0's at N>1) as DIR/<field>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.workload != "cfg2":
+        ap.error("--dump-outputs needs the cfg2 workload (the timed steps)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
