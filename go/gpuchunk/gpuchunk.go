@@ -514,6 +514,17 @@ func (b *Batch) BlobEncode(off, length []uint64) ([][]byte, error) {
 // keeps a compressed payload only then).  The frames are built on the GPU from RLE and raw blocks -- they remove
 // the zero runs of disk images and sparse files; data without such runs stays uncompressed.
 func (b *Batch) BlobEncodeZ(off, length []uint64) ([][]byte, error) {
+	return b.blobEncodeZstd(off, length, false)
+}
+
+// BlobEncodeLZ is BlobEncodeZ whose frames also hold zstd Compressed_Blocks from the GPU's greedy LZ parse wherever
+// those are smaller than the block: text, logs and repeated records shrink too.  It costs more GPU time per byte than
+// BlobEncodeZ and compresses less than zstd level 1 (no Huffman literals, predefined FSE tables, block-local matches).
+func (b *Batch) BlobEncodeLZ(off, length []uint64) ([][]byte, error) {
+	return b.blobEncodeZstd(off, length, true)
+}
+
+func (b *Batch) blobEncodeZstd(off, length []uint64, lz bool) ([][]byte, error) {
 	n := len(off)
 	if n == 0 {
 		return nil, nil
@@ -528,7 +539,12 @@ func (b *Batch) BlobEncodeZ(off, length []uint64) ([][]byte, error) {
 		total += uint64(C.pbsgpu_blob_size(C.uint64_t(length[i])))
 	}
 	out := make([]byte, total+1)
-	rc := C.pbsgpu_blob_encode_batch_z(b.e.ctx, b.buf, &o[0], &l[0], C.uint32_t(n), (*C.uint8_t)(unsafe.Pointer(&out[0])), &oo[0], &ol[0], nil)
+	var rc C.int
+	if lz {
+		rc = C.pbsgpu_blob_encode_batch_lz(b.e.ctx, b.buf, &o[0], &l[0], C.uint32_t(n), (*C.uint8_t)(unsafe.Pointer(&out[0])), &oo[0], &ol[0], nil)
+	} else {
+		rc = C.pbsgpu_blob_encode_batch_z(b.e.ctx, b.buf, &o[0], &l[0], C.uint32_t(n), (*C.uint8_t)(unsafe.Pointer(&out[0])), &oo[0], &ol[0], nil)
+	}
 	if err := b.e.err(rc); err != nil {
 		return nil, err
 	}

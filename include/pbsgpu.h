@@ -281,6 +281,15 @@ int pbsgpu_blob_encode_batch(pbsgpu_ctx *ctx, const void *base, const uint64_t *
  * same input (no two zstd encoders are). */
 int pbsgpu_blob_encode_batch_z(pbsgpu_ctx *ctx, const void *base, const uint64_t *off, const uint64_t *len, uint32_t n,
                                uint8_t *out, const uint64_t *out_off, uint64_t *out_len, uint32_t *crc_out);
+/* pbsgpu_blob_encode_batch_z plus zstd's match stage (K9): the same arguments, reservation and blob-level rule, and the
+ * same frame and 128 KiB block grid, but a block that is not one repeated byte becomes a Compressed_Block wherever
+ * that is smaller than the block (Raw_Block otherwise).  The Compressed_Block holds the sequences of a greedy LZ parse
+ * confined to its own block (4-byte minimum match, 2^14-entry hash table) with Raw_Literals and the three predefined
+ * FSE tables; it omits Huffman-coded literals, FSE-compressed or repeated tables, repeat offsets, lazy parsing and
+ * matches across blocks, so it compresses less than libzstd level 1 and costs more GPU time than the _z call.  Text,
+ * logs and repeated records shrink; any zstd decoder reads the result. */
+int pbsgpu_blob_encode_batch_lz(pbsgpu_ctx *ctx, const void *base, const uint64_t *off, const uint64_t *len, uint32_t n,
+                                uint8_t *out, const uint64_t *out_off, uint64_t *out_len, uint32_t *crc_out);
 
 /* ---- f2 ("next" row): the commit walk's per-file content hash ----------------------------------
  * emitBackedFile tees every new file through `xxh3.New()` and keeps `h.Sum64()` (reference

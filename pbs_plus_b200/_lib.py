@@ -79,7 +79,7 @@ SYMBOLS = [
     "pbsgpu_set_destroy", "pbsgpu_set_insert", "pbsgpu_set_probe", "pbsgpu_set_count", "pbsgpu_set_seed_didx",
     "pbsgpu_set_allgather", "pbsgpu_nccl_unique_id", "pbsgpu_nccl_comm_create", "pbsgpu_nccl_comm_destroy",
     "pbsgpu_didx_size", "pbsgpu_didx_build", "pbsgpu_didx_parse", "pbsgpu_crc32_batch", "pbsgpu_blob_header",
-    "pbsgpu_blob_size", "pbsgpu_blob_encode_batch", "pbsgpu_blob_encode_batch_z",
+    "pbsgpu_blob_size", "pbsgpu_blob_encode_batch", "pbsgpu_blob_encode_batch_z", "pbsgpu_blob_encode_batch_lz",
     "pbsgpu_xxh3_batch", "pbsgpu_chunk_digest_batch_xxh3",
     "pbsgpu_host_alloc", "pbsgpu_host_free", "pbsgpu_corpus_fill",
 ]
@@ -145,6 +145,7 @@ def lib() -> C.CDLL:
     L.pbsgpu_blob_size.restype = C.c_uint64
     L.pbsgpu_blob_encode_batch.argtypes = [vp, vp, vp, vp, C.c_uint32, vp, vp, vp]
     L.pbsgpu_blob_encode_batch_z.argtypes = [vp, vp, vp, vp, C.c_uint32, vp, vp, vp, vp]
+    L.pbsgpu_blob_encode_batch_lz.argtypes = [vp, vp, vp, vp, C.c_uint32, vp, vp, vp, vp]
     L.pbsgpu_set_create.argtypes = [vp, C.c_uint64, C.POINTER(vp)]
     L.pbsgpu_set_destroy.argtypes = [vp]
     L.pbsgpu_set_destroy.restype = None

@@ -17,7 +17,7 @@ CSRC = HERE / "csrc"
 OBJ = HERE / "_obj"
 LIB = HERE / "libpbsgpu.so"
 SOURCES = ["scan.cu", "resolve.cu", "sha256.cu", "digestset.cu", "crc32.cu", "xxh3.cu", "corpus.cu", "capi.cu", "capi_set.cu",
-           "capi_stream.cu", "capi_aux.cu", "zframe.cu"]
+           "capi_stream.cu", "capi_aux.cu", "zframe.cu", "zlz.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

@@ -90,7 +90,9 @@ extern "C" int pbsgpu_crc32_batch(pbsgpu_ctx *ctx, const void *base, const uint6
         std::vector<uint8_t> h(crc_tables_bytes());
         crc_fill_tables_host(h.data());
         CK(cudaMalloc(&ctx->d_crc_tables, h.size()));
-        CK(cudaMemcpy(ctx->d_crc_tables, h.data(), h.size(), cudaMemcpyHostToDevice));
+        // a pageable cudaMemcpy may return before its DMA lands, and the kernels run on non-blocking streams: wait here
+        CK(cudaMemcpyAsync(ctx->d_crc_tables, h.data(), h.size(), cudaMemcpyHostToDevice, st));
+        CK(cudaStreamSynchronize(st));
     }
     const int crc_variant = ctx->crc_variant;   // 0 = TMA-tiled kernel (default), 1 = simple lane-strided kernel (PBSGPU_CRC_VARIANT at open)
     uint64_t hi = 0;
@@ -164,11 +166,12 @@ extern "C" int pbsgpu_blob_encode_batch(pbsgpu_ctx *ctx, const void *base, const
 
 // f3, compressed form: DataBlobs whose payload is a zstd frame when that is smaller than the raw bytes (upstream
 // `DataBlob::encode` keeps the compressed form only then).  The frame is built on the device from RLE_Blocks (128 KiB
-// blocks of one repeated byte) and Raw_Blocks (zframe.cu) -- no match / entropy stage; the CRC (K6) covers the frame.
+// blocks of one repeated byte) and Raw_Blocks (zframe.cu), and with `lz` also from Compressed_Blocks (K9, zlz.cu) where
+// those come out smaller than the block; the CRC (K6) covers the frame.
 static const uint8_t BLOB_MAGIC_COMPRESSED[8] = {49, 185, 88, 66, 111, 182, 163, 127};
 
-extern "C" int pbsgpu_blob_encode_batch_z(pbsgpu_ctx *ctx, const void *base, const uint64_t *off, const uint64_t *len, uint32_t n,
-                                          uint8_t *out, const uint64_t *out_off, uint64_t *out_len, uint32_t *crc_out) {
+static int blob_encode_zstd(pbsgpu_ctx *ctx, const void *base, const uint64_t *off, const uint64_t *len, uint32_t n,
+                            uint8_t *out, const uint64_t *out_off, uint64_t *out_len, uint32_t *crc_out, bool lz) {
     if (!ctx || (n && (!off || !len || !out || !out_off || !out_len || !base))) return PBSGPU_EINVAL;
     Guard g(ctx);
     if (n == 0) return PBSGPU_OK;
@@ -202,6 +205,42 @@ extern "C" int pbsgpu_blob_encode_batch_z(pbsgpu_ctx *ctx, const void *base, con
         if (e == cudaSuccess) e = es;
         if (e != cudaSuccess) { (void)cudaGetLastError(); return fail(ctx, PBSGPU_ECUDA, "zstd block scan: %s", cudaGetErrorString(e)); }
     }
+    // K9: every block that is not one repeated byte -> a Compressed_Block in its slot, or raw (lz_info 0)
+    std::vector<uint32_t> lz_info(lz ? n_blocks : 0, 0), lz_slot(lz ? n_blocks : 0, 0);
+    std::vector<uint64_t> l_src;
+    std::vector<uint32_t> l_size;
+    for (uint32_t i = 0; lz && i < n; i++)
+        for (uint64_t b = 0; b < blk_first[i + 1] - blk_first[i]; b++)
+            if (!(flags[blk_first[i] + b] & 0x100u)) {
+                lz_slot[blk_first[i] + b] = (uint32_t)l_src.size();
+                l_src.push_back(off[i] + b * ZFRAME_BLOCK);
+                l_size.push_back((uint32_t)std::min<uint64_t>(ZFRAME_BLOCK, len[i] - b * ZFRAME_BLOCK));
+            }
+    const uint32_t nl = (uint32_t)l_src.size();
+    Scoped lz_stage(ctx->dev, nl ? (uint64_t)nl * ZLZ_SLOT : 0);
+    if (nl) {
+        if (!lz_stage) return fail(ctx, PBSGPU_ENOMEM, "match stage output of %llu bytes failed", (unsigned long long)nl * ZLZ_SLOT);
+        // 16 walking warps per SM (K9b); the pass's scratch is ~528 KiB per block, ~1 GiB at 124 bulk SMs
+        const uint32_t pass = std::min<uint32_t>(nl, 16 * (uint32_t)ctx->sm_count);
+        Scoped d_src(ctx->dev, nl * 8ull), d_size(ctx->dev, nl * 4ull), d_info(ctx->dev, nl * 4ull),
+            scratch(ctx->dev, pass * zlz_scratch_bytes_per_block());
+        if (!d_src || !d_size || !d_info || !scratch) return fail(ctx, PBSGPU_ENOMEM, "device allocation failed");
+        std::vector<uint32_t> info(nl);
+        cudaError_t e = cudaMemcpyAsync(d_src.p, l_src.data(), nl * 8ull, cudaMemcpyHostToDevice, st);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(d_size.p, l_size.data(), nl * 4ull, cudaMemcpyHostToDevice, st);
+        if (e == cudaSuccess) e = launch_zlz(dbase, d_src.as<uint64_t>(), d_size.as<uint32_t>(), nl, lz_stage.as<uint8_t>(), d_info.as<uint32_t>(), scratch.p, pass, st);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(info.data(), d_info.p, nl * 4ull, cudaMemcpyDeviceToHost, st);
+        cudaError_t es = cudaStreamSynchronize(st);
+        if (e == cudaSuccess) e = es;
+        if (e != cudaSuccess) { (void)cudaGetLastError(); return fail(ctx, PBSGPU_ECUDA, "zstd match stage: %s", cudaGetErrorString(e)); }
+        for (uint64_t g = 0; g < n_blocks; g++)
+            if (!(flags[g] & 0x100u)) lz_info[g] = info[lz_slot[g]];
+    }
+    // per block: 1 byte (RLE), the Compressed_Block (K9) or the raw bytes
+    auto content_bytes = [&](uint64_t g, uint64_t size) -> uint64_t {
+        if (flags[g] & 0x100u) return 1;
+        return lz && lz_info[g] ? (lz_info[g] & 0xFFFFFFu) : size;
+    };
     // frame sizes; the chunks that come out smaller get a place in the stage and one emit entry per block
     std::vector<uint8_t> comp(n, 0);
     std::vector<uint64_t> frame_len(n, 0), frame_off, content, e_src, e_dst;
@@ -212,7 +251,7 @@ extern "C" int pbsgpu_blob_encode_batch_z(pbsgpu_ctx *ctx, const void *base, con
         uint64_t fl = ZFRAME_HEADER;
         for (uint64_t b = 0; b < nb; b++) {
             const uint64_t size = std::min<uint64_t>(ZFRAME_BLOCK, len[i] - b * ZFRAME_BLOCK);
-            fl += 3 + ((flags[blk_first[i] + b] & 0x100u) ? 1 : size);
+            fl += 3 + content_bytes(blk_first[i] + b, size);
         }
         frame_len[i] = fl;
         if (len[i] == 0 || fl >= len[i]) continue;
@@ -223,12 +262,16 @@ extern "C" int pbsgpu_blob_encode_batch_z(pbsgpu_ctx *ctx, const void *base, con
         uint64_t pos = cursor + ZFRAME_HEADER;
         for (uint64_t b = 0; b < nb; b++) {
             const uint64_t size = std::min<uint64_t>(ZFRAME_BLOCK, len[i] - b * ZFRAME_BLOCK);
-            const uint32_t f = flags[blk_first[i] + b];
-            const bool rle = (f & 0x100u) != 0;
-            e_src.push_back(off[i] + b * ZFRAME_BLOCK);
+            const uint64_t g = blk_first[i] + b;
+            const uint32_t f = flags[g];
+            const bool rle = (f & 0x100u) != 0, cmp = !rle && lz && lz_info[g];
+            const uint64_t bytes = content_bytes(g, size);
+            // Block_Size is the repeat count for RLE, the content size otherwise
+            e_src.push_back(cmp ? (uint64_t)lz_slot[g] * ZLZ_SLOT + (lz_info[g] >> 24) : off[i] + b * ZFRAME_BLOCK);
             e_dst.push_back(pos);
-            e_hdr.push_back((uint32_t)(b + 1 == nb) | ((rle ? 1u : 0u) << 1) | ((uint32_t)size << 3) | ((f & 0xFFu) << 24));
-            pos += 3 + (rle ? 1 : size);
+            e_hdr.push_back((uint32_t)(b + 1 == nb) | ((rle ? 1u : cmp ? 2u : 0u) << 1) | ((uint32_t)(rle ? size : bytes) << 3) |
+                            ((f & 0xFFu) << 24));
+            pos += 3 + bytes;
         }
         cursor = (pos + 15) & ~15ull;
     }
@@ -246,7 +289,7 @@ extern "C" int pbsgpu_blob_encode_batch_z(pbsgpu_ctx *ctx, const void *base, con
         if (e == cudaSuccess) e = cudaMemcpyAsync(d_foff.p, frame_off.data(), nc * 8, cudaMemcpyHostToDevice, st);
         if (e == cudaSuccess) e = cudaMemcpyAsync(d_clen.p, content.data(), nc * 8, cudaMemcpyHostToDevice, st);
         if (e == cudaSuccess) e = launch_zframe_hdr(stage.as<uint8_t>(), d_foff.as<uint64_t>(), d_clen.as<uint64_t>(), nc, st);
-        if (e == cudaSuccess) e = launch_zframe_emit(dbase, stage.as<uint8_t>(), d_src.as<uint64_t>(), d_dst.as<uint64_t>(), d_hdr.as<uint32_t>(), ne, st);
+        if (e == cudaSuccess) e = launch_zframe_emit(dbase, nl ? lz_stage.as<uint8_t>() : nullptr, stage.as<uint8_t>(), d_src.as<uint64_t>(), d_dst.as<uint64_t>(), d_hdr.as<uint32_t>(), ne, st);
         cudaError_t es = cudaStreamSynchronize(st);
         if (e == cudaSuccess) e = es;
         if (e != cudaSuccess) { (void)cudaGetLastError(); return fail(ctx, PBSGPU_ECUDA, "zstd frame emit: %s", cudaGetErrorString(e)); }
@@ -292,6 +335,16 @@ extern "C" int pbsgpu_blob_encode_batch_z(pbsgpu_ctx *ctx, const void *base, con
     return PBSGPU_OK;
 }
 
+extern "C" int pbsgpu_blob_encode_batch_z(pbsgpu_ctx *ctx, const void *base, const uint64_t *off, const uint64_t *len, uint32_t n,
+                                          uint8_t *out, const uint64_t *out_off, uint64_t *out_len, uint32_t *crc_out) {
+    return blob_encode_zstd(ctx, base, off, len, n, out, out_off, out_len, crc_out, false);
+}
+
+extern "C" int pbsgpu_blob_encode_batch_lz(pbsgpu_ctx *ctx, const void *base, const uint64_t *off, const uint64_t *len, uint32_t n,
+                                           uint8_t *out, const uint64_t *out_off, uint64_t *out_len, uint32_t *crc_out) {
+    return blob_encode_zstd(ctx, base, off, len, n, out, out_off, out_len, crc_out, true);
+}
+
 // ---------------------------------------------------------------------------
 // f2: XXH3-64 of n byte ranges (the commit walk's per-file content hash, commit.go:717-725, :957-976).
 // Blocks are hashed in passes of at most PBSGPU_XXH3_CAP_BLOCKS (default 8 Mi = 8 GiB of input, 512 MiB
@@ -312,7 +365,9 @@ int pbsgpu_xxh3_enqueue(pbsgpu_ctx *ctx, const uint8_t *dbase, const uint64_t *o
         std::vector<uint8_t> h(xxh3_tables_bytes());
         xxh3_fill_tables_host(h.data());
         CK(cudaMalloc(&ctx->d_xxh_tab, h.size()));
-        CK(cudaMemcpy(ctx->d_xxh_tab, h.data(), h.size(), cudaMemcpyHostToDevice));
+        // as for the CRC tables: the table must have landed before any stream's kernel reads it
+        CK(cudaMemcpyAsync(ctx->d_xxh_tab, h.data(), h.size(), cudaMemcpyHostToDevice, st));
+        CK(cudaStreamSynchronize(st));
     }
     const uint64_t cap_blocks = ctx->xxh3_cap_blocks;
     uint64_t total_all = 0, max_nb = 0, n_long = 0;

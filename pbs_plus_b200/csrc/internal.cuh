@@ -123,9 +123,23 @@ constexpr uint32_t ZFRAME_BLOCK = 128u * 1024u;   // Block_Maximum_Size
 constexpr uint32_t ZFRAME_HEADER = 13;            // magic 4 + descriptor 1 + content size 8
 cudaError_t launch_zblock_scan(const uint8_t *base, const uint64_t *off, const uint64_t *len, const uint64_t *blk_first,
                                uint32_t n, uint64_t n_blocks, uint32_t *flags, cudaStream_t st);
-cudaError_t launch_zframe_emit(const uint8_t *base, uint8_t *stage, const uint64_t *src_off, const uint64_t *dst_off,
-                               const uint32_t *hdr, uint64_t n_entries, cudaStream_t st);
+// Block_Type 2 (Compressed_Block) entries copy from `lz` (K9's slots) instead of `base`; NULL when there are none
+cudaError_t launch_zframe_emit(const uint8_t *base, const uint8_t *lz, uint8_t *stage, const uint64_t *src_off,
+                               const uint64_t *dst_off, const uint32_t *hdr, uint64_t n_entries, cudaStream_t st);
 cudaError_t launch_zframe_hdr(uint8_t *stage, const uint64_t *frame_off, const uint64_t *content_len, uint32_t n, cudaStream_t st);
+
+// ---- f3: zstd match stage (K9, zlz.cu) ------------------------------------------------------
+// The greedy parse's constants; oracle/zstd_lz.py (LZ_HLOG, LZ_SEG, LZ_MINMATCH) states the same parse.
+constexpr int ZLZ_HLOG = 14;          // hash table of 2^14 positions
+constexpr uint32_t ZLZ_SEG = 1024;    // positions look up only earlier segments of this length
+constexpr uint32_t ZLZ_MINMATCH = 4;
+constexpr uint32_t ZLZ_SLOT = ZFRAME_BLOCK + 64;   // bytes per block in K9's output (a kept block is < its input)
+// Block b of the list (blk_src[b] bytes into base, blk_size[b] <= ZFRAME_BLOCK bytes) -> Block_Content at
+// slots + b * ZLZ_SLOT + (info[b] >> 24) of (info[b] & 0xFFFFFF) bytes, or info[b] = 0: keep the block raw.  The blocks
+// go in passes of pass_blocks; `scratch` holds zlz_scratch_bytes_per_block() per block of a pass.
+uint64_t zlz_scratch_bytes_per_block();
+cudaError_t launch_zlz(const uint8_t *base, const uint64_t *blk_src, const uint32_t *blk_size, uint32_t n_blk, uint8_t *slots,
+                       uint32_t *info, void *scratch, uint32_t pass_blocks, cudaStream_t st);
 
 // ---- digest set (K4) ----------------------------------------------------------------
 struct SetTable {

@@ -11,6 +11,7 @@
 //                       first 16 KiB that disagrees -- HBM traffic ~ the constant bytes + 16 KiB per other block
 //   K8b k_zframe_emit : one CTA per block of the chunks that come out smaller: 3-byte Block_Header + 1 byte (RLE) or
 //                       + the raw bytes (funnel-shifted 4-byte copy: the 3-byte headers misalign source and target)
+//                       or + a Compressed_Block's content from K9's slots (zlz.cu)
 //   K8c k_zframe_hdr  : the 13-byte Frame_Header of each such chunk
 #include "internal.cuh"
 
@@ -60,8 +61,8 @@ cudaError_t launch_zblock_scan(const uint8_t *base, const uint64_t *off, const u
 }
 
 // hdr[e]: bits 0..23 = the Block_Header (Last_Block | Block_Type << 1 | Block_Size << 3), bits 24..31 = the RLE byte
-__global__ void __launch_bounds__(256) k_zframe_emit(const uint8_t *base, uint8_t *stage, const uint64_t *src_off,
-                                                     const uint64_t *dst_off, const uint32_t *hdr) {
+__global__ void __launch_bounds__(256) k_zframe_emit(const uint8_t *base, const uint8_t *lz, uint8_t *stage,
+                                                     const uint64_t *src_off, const uint64_t *dst_off, const uint32_t *hdr) {
     const uint64_t e = blockIdx.x;
     const uint32_t h = hdr[e];
     uint8_t *d = stage + dst_off[e];
@@ -72,7 +73,7 @@ __global__ void __launch_bounds__(256) k_zframe_emit(const uint8_t *base, uint8_
         return;
     }
     uint8_t *dst = d + 3;
-    const uint8_t *src = base + src_off[e];
+    const uint8_t *src = (type == 2 ? lz : base) + src_off[e];
     uint32_t head = (uint32_t)((4 - ((uintptr_t)dst & 3)) & 3);
     if (head > size) head = size;
     if (threadIdx.x < head) dst[threadIdx.x] = src[threadIdx.x];
@@ -87,11 +88,11 @@ __global__ void __launch_bounds__(256) k_zframe_emit(const uint8_t *base, uint8_
         dst32[w] = __funnelshift_r(a0, a1, sh);
     }
 }
-cudaError_t launch_zframe_emit(const uint8_t *base, uint8_t *stage, const uint64_t *src_off, const uint64_t *dst_off,
-                               const uint32_t *hdr, uint64_t n_entries, cudaStream_t st) {
+cudaError_t launch_zframe_emit(const uint8_t *base, const uint8_t *lz, uint8_t *stage, const uint64_t *src_off,
+                               const uint64_t *dst_off, const uint32_t *hdr, uint64_t n_entries, cudaStream_t st) {
     if (n_entries == 0) return cudaSuccess;
     if (n_entries >= (1ull << 31)) return cudaErrorInvalidValue;
-    k_zframe_emit<<<(unsigned)n_entries, 256, 0, st>>>(base, stage, src_off, dst_off, hdr);
+    k_zframe_emit<<<(unsigned)n_entries, 256, 0, st>>>(base, lz, stage, src_off, dst_off, hdr);
     return cudaGetLastError();
 }
 

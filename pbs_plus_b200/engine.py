@@ -248,6 +248,14 @@ class Engine:
     def blob_encode_batch_z(self, base, off, length):
         """DataBlobs with a zstd payload where that is smaller (RLE / raw block frames, pbsgpu_blob_encode_batch_z)
         -> list of n `bytes` blobs, crc[n]."""
+        return self._blob_encode_zstd(self._L.pbsgpu_blob_encode_batch_z, base, off, length)
+
+    def blob_encode_batch_lz(self, base, off, length):
+        """blob_encode_batch_z whose frames also hold Compressed_Blocks from the GPU's greedy LZ parse where those are
+        smaller (pbsgpu_blob_encode_batch_lz) -> list of n `bytes` blobs, crc[n]."""
+        return self._blob_encode_zstd(self._L.pbsgpu_blob_encode_batch_lz, base, off, length)
+
+    def _blob_encode_zstd(self, fn, base, off, length):
         o, l = self._offlen(off, length)
         sizes = l + np.uint64(12)
         boff = np.zeros(len(o) + 1, dtype=np.uint64)
@@ -255,8 +263,8 @@ class Engine:
         out = np.zeros(max(1, int(boff[-1])), dtype=np.uint8)
         blen = np.zeros(len(o), dtype=np.uint64)
         crc = np.zeros(len(o), dtype=np.uint32)
-        self._ck(self._L.pbsgpu_blob_encode_batch_z(self._h, _ptr(base), o.ctypes.data, l.ctypes.data, len(o),
-                                                    out.ctypes.data, boff.ctypes.data, blen.ctypes.data, crc.ctypes.data))
+        self._ck(fn(self._h, _ptr(base), o.ctypes.data, l.ctypes.data, len(o), out.ctypes.data, boff.ctypes.data,
+                    blen.ctypes.data, crc.ctypes.data))
         return [out[int(boff[i]): int(boff[i]) + int(blen[i])].tobytes() for i in range(len(o))], crc
 
     def blob_header(self, crc: int) -> bytes:

@@ -58,6 +58,9 @@ class DedupWriter:
     # chunks of a flush by ONE pbsgpu_blob_encode_batch_z call (zstd frame where smaller, CRC-32 from the GPU)
     upload_blob: Callable[[bytes, bytes], None] | None = None
     batch_bytes: int = 1 << 30
+    # "rle": frames of RLE / raw blocks (pbsgpu_blob_encode_batch_z); "lz": also Compressed_Blocks from the GPU's match
+    # stage (pbsgpu_blob_encode_batch_lz) -- smaller blobs for text-like data at more GPU time per byte
+    blob_codec: str = "rle"
     index: list[IndexRecord] = field(default_factory=list)
     # relPath -> XXH3-64 of the file as uploaded: commitWalkState.backedHashes (commit.go:187, :725), computed on the
     # GPU from the same staged bytes instead of through an io.TeeReader on the host
@@ -65,6 +68,10 @@ class DedupWriter:
     _pending: list[tuple[Entry, np.ndarray]] = field(default_factory=list)
     _pending_bytes: int = 0
     _finished: bool = False
+
+    def __post_init__(self) -> None:
+        if self.blob_codec not in ("rle", "lz"):
+            raise ValueError(f"transfer: unknown blob_codec {self.blob_codec!r} (want 'rle' or 'lz')")
 
     def WriteEntryReader(self, entry: Entry, reader: BinaryIO, size: int) -> None:
         """Pulls exactly `size` bytes from `reader` (error if it yields fewer, like io.ReadFull)."""
@@ -105,7 +112,8 @@ class DedupWriter:
         if self.upload_blob is not None and new_chunks:
             boff = np.array([int(offs[i]) + s0 for _, i, s0, _ in new_chunks], dtype=np.uint64)
             blen = np.array([e0 - s0 for _, _, s0, e0 in new_chunks], dtype=np.uint64)
-            blobs, _crc = self.engine.blob_encode_batch_z(buf, boff, blen)
+            encode = self.engine.blob_encode_batch_lz if self.blob_codec == "lz" else self.engine.blob_encode_batch_z
+            blobs, _crc = encode(buf, boff, blen)
             for (d, _i, _s, _e), blob in zip(new_chunks, blobs):
                 self.upload_blob(d, blob)
         self._pending, self._pending_bytes = [], 0
@@ -255,14 +263,16 @@ class PayloadStreamWriter:
 
 
 def NewRemoteDedupSplitArchiveWriter(engine: Engine, config: Cfg, known: DigestSet | None = None,
-                                     orig_payload_idx: bytes | None = None, upload=None, upload_blob=None) -> DedupWriter:
+                                     orig_payload_idx: bytes | None = None, upload=None, upload_blob=None,
+                                     blob_codec: str = "rle") -> DedupWriter:
     """commit.go:329.  `orig_payload_idx` = bytes of the previous .ppxar.didx (commit.go:324-328):
-    its digests seed the known set, so unchanged chunks are not uploaded again."""
+    its digests seed the known set, so unchanged chunks are not uploaded again.  `blob_codec` picks the DataBlob
+    encoder of `upload_blob` (DedupWriter.blob_codec)."""
     if orig_payload_idx:
         if known is None:
             known = engine.digest_set()
         known.seed_didx(orig_payload_idx)
-    return DedupWriter(engine, config, known, upload, upload_blob)
+    return DedupWriter(engine, config, known, upload, upload_blob, blob_codec=blob_codec)
 
 
 def verifyBackedFileHashes(engine: Engine, open_file: Callable[[str], BinaryIO], hashes: dict[str, int],
